@@ -2,6 +2,7 @@
 """bench.py -- forward+backward Gaussians/s of the strand-aligned rasterizer hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl mine|reference] [--mode native|render|render_hair]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the one `metric` is quoted on): 500 000 synthetic strand-aligned
 Gaussians (SURVEY.md 8d scene "strands(5000)"), 1920x1080, one ring camera per step, forward +
@@ -56,7 +57,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--ref-steps", type=int, default=10)
-    ap.add_argument("--repeats", type=int, default=5, help="how many times the timed K-step window is repeated (median reported)")
+    ap.add_argument("--repeats", type=int, default=1, help="how many times the timed K-step window is repeated (median reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (image, radii, gradients) as DIR/<name>.npy")
     ap.add_argument("--collective", default="auto", choices=["auto", "peer-mc", "peer-nomc", "nccl"],
                     help="N>1: gh_allreduce_p2p over symmetric memory (auto: peer ld/st up to 4 GPUs, NVLS multimem from 8) or NCCL")
     return ap.parse_args()
@@ -137,6 +140,32 @@ def algorithmic_bytes(P, R, W, H, T, mode):
     }
     path = (400 if native else 344) * P + 52 * R + 96 * W * H + 24 * T
     return stage, path
+
+
+DUMP_BYTES = 60 << 20
+# positions of the rasterizer's 9 gradients in the tuple `rasterize_gaussians_backward` returns
+GRAD_TUPLE = ("means2D", "colors", "opacity", "means3D", "cov3D", "conic", "sh", "scales", "rotations")
+
+
+def dump_outputs(out_dir, last):
+    """The arrays the last timed step handed to its caller -- the rendered image, radii, num_rendered and every
+    gradient -- as float32 `.npy` files (num_rendered float64).  An array larger than its share of DUMP_BYTES is
+    replaced by the values at a fixed, seeded set of positions, so that two builds can be compared file by file."""
+    import numpy as np
+    import torch
+    grads = last["views"] if "views" in last else dict(zip(GRAD_TUPLE, last["grads"]))
+    arrays = {"color": last["color"], "radii": last["radii"]}
+    arrays.update({f"grad_{k}": v for k, v in grads.items() if v is not None and v.numel() > 0})
+    cap = DUMP_BYTES // 4 // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        v = t.detach().reshape(-1).float()
+        if v.numel() > cap:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            v = v[idx.to(v.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy())
+    np.save(os.path.join(out_dir, "num_rendered.npy"), np.array([float(last["R"])], np.float64))
+    log(f"[bench] outputs of the last timed step written to {out_dir} ({len(arrays) + 1} arrays)")
 
 
 def main():
@@ -265,6 +294,7 @@ def main():
     def step(i, mod=native, arena=(args.impl == "mine"), plist=None):
         fw, kw, s, e, g = (plist or packed)[i % len(packed)]
         R, color, radii, geom, binning, img = mod.rasterize_gaussians(*fw)
+        last["color"], last["radii"] = color, radii
         bw = (s["bg"], kw["means3D"], radii, g("colors_precomp"), g("scales"), g("rotations"), s["scale_modifier"],
               g("cov3D_precomp"), g("conic_precomp"), s["viewmatrix"], s["projmatrix"], s["tanfovx"], s["tanfovy"],
               dL, e, s["sh_degree"], s["campos"], geom, R, binning, img, False)
@@ -321,6 +351,8 @@ def main():
             gpu_launches = int(_capi.load().gh_kernel_launch_count() - launches0)
     clocks = sampler.stop() if rank == 0 else None
     ms_total = statistics.median(windows)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     ms_per_step = ms_total / args.steps
     n_eff = N if args.impl == "mine" else 1       # reference arm: rank 0 alone runs (one GPU's worth of work)
     value = (args.steps * P * n_eff) / (ms_total * 1e-3)

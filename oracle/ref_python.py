@@ -129,10 +129,14 @@ def make_gaussian_model(scene: dict, device, sh_degree: int = 3, active_sh_degre
     """A real reference `GaussianModel` (scene/gaussian_model.py:45) whose parameters are set from a seeded
     synthetic scene the way `create_from_pcd` / `load_ply` set them (:409-419, :569-577): raw log-scales,
     raw quaternions, logit opacities / labels, log orientation confidences."""
+    from scene.gaussian_model import GaussianModel
+    return fill_gaussian_model(GaussianModel(sh_degree), scene, device, active_sh_degree)
+
+
+def fill_gaussian_model(pc, scene: dict, device, active_sh_degree: int = 3):
+    """Set the parameters of `pc` (a GaussianModel, or any object with its attribute names) from a seeded scene."""
     import torch
     from torch import nn
-    from scene.gaussian_model import GaussianModel
-    pc = GaussianModel(sh_degree)
     P = lambda t: nn.Parameter(t.detach().clone().to(device).contiguous().requires_grad_(True))  # noqa: E731
     logit = lambda p: torch.log(p / (1 - p))  # noqa: E731
     pc._xyz = P(scene["xyz"])
@@ -146,6 +150,12 @@ def make_gaussian_model(scene: dict, device, sh_degree: int = 3, active_sh_degre
     pc.active_sh_degree = active_sh_degree
     pc.max_radii2D = torch.zeros(pc._xyz.shape[0], device=device)
     return pc
+
+
+def plain_gaussian_model(scene: dict, device, sh_degree: int = 3):
+    """The GaussianModel attributes that this repository's renderer and densification read, on a plain namespace
+    (no reference sources needed)."""
+    return fill_gaussian_model(types.SimpleNamespace(max_sh_degree=sh_degree), scene, device, sh_degree)
 
 
 MODEL_PARAMS = ("_xyz", "_features_dc", "_features_rest", "_scaling", "_rotation", "_opacity", "_label", "_orient_conf")

@@ -115,6 +115,118 @@ def rel_err(a: torch.Tensor, b: torch.Tensor) -> float:
     return d / nb
 
 
+# ------------------------------------------------------------------ stored reference results (tests/golden/reference/*.npz)
+# The reference's outputs of the GPU parity tests are stored as fingerprints small enough to commit
+# (tests/golden/make_golden_reference.py writes them): a digest of the bytes for the bit-exact checks, the
+# exact norm and max|x|, a count sketch (the norm of a difference is estimated over EVERY element) and the
+# values at a few seeded positions (element-wise checks).
+SKETCH = 16
+SAMPLE = 8
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+
+
+def _np(x) -> np.ndarray:
+    if isinstance(x, torch.Tensor):
+        x = x.detach().cpu().contiguous().numpy()
+    return np.ascontiguousarray(np.asarray(x))
+
+
+def digest(x) -> bytes:
+    import hashlib
+    return hashlib.sha256(_np(x).tobytes()).digest()[:16]
+
+
+_hashes = {}
+
+
+def _hash(n: int, device):
+    """Seeded bucket, sign and sample position of every element of an n-element array."""
+    key = (n, str(device))
+    if key not in _hashes:
+        g = torch.Generator().manual_seed(20240917)
+        bucket = torch.randint(0, SKETCH, (n,), generator=g)
+        sign = (torch.randint(0, 2, (n,), generator=g) * 2 - 1).double()
+        pos = torch.randint(0, max(n, 1), (SAMPLE,), generator=g)
+        _hashes.clear()
+        _hashes[key] = (bucket.to(device), sign.to(device), pos)
+    return _hashes[key]
+
+
+def _flat64(x) -> torch.Tensor:
+    if not isinstance(x, torch.Tensor):
+        return torch.from_numpy(_np(x).astype(np.float64).reshape(-1))
+    return x.detach().reshape(-1).double()
+
+
+def sketch(x) -> torch.Tensor:
+    v = _flat64(x)
+    bucket, sign, _ = _hash(v.numel(), v.device)
+    return torch.zeros(SKETCH, dtype=torch.float64, device=v.device).index_add_(0, bucket, v * sign).cpu()
+
+
+def fingerprint(x) -> tuple:
+    """(shape, digest, [numel, norm, max|x|, sketch..., sample...]) of a tensor or array."""
+    v = _flat64(x)
+    n = v.numel()
+    sample = torch.zeros(SAMPLE, dtype=torch.float64)
+    if n:
+        sample = v[_hash(n, v.device)[2].to(v.device)].cpu()
+    stats = [float(n), v.norm().item() if n else 0.0, v.abs().max().item() if n else 0.0]
+    row = np.concatenate([np.array(stats), sketch(v).numpy(), sample.numpy()])
+    return tuple(_np(x).shape), digest(x), row
+
+
+def save_golden(path: str, records: dict) -> None:
+    """records: key -> tensor/array (the reference's result)."""
+    keys = sorted(records)
+    fps = [fingerprint(records[k]) for k in keys]
+    np.savez_compressed(path, keys=np.array(keys), shapes=np.array([",".join(map(str, f[0])) for f in fps]),
+                        digests=np.frombuffer(b"".join(f[1] for f in fps), np.uint8).reshape(len(keys), 16),
+                        rows=np.stack([f[2] for f in fps]))
+
+
+class Ref:
+    """A reference tensor known by its fingerprint."""
+
+    def __init__(self, shape, dig, row):
+        self.shape = shape
+        self.digest = dig
+        self.numel, self.norm, self.absmax = int(row[0]), float(row[1]), float(row[2])
+        self.sketch = torch.from_numpy(row[3:3 + SKETCH].copy())
+        self.sample = torch.from_numpy(row[3 + SKETCH:].copy())
+
+    def equal(self, x) -> bool:
+        """Bit-identical (same shape, dtype and bytes)."""
+        return tuple(_np(x).shape) == self.shape and digest(x) == self.digest
+
+    def rel_err(self, x) -> float:
+        """||x - ref|| / ||ref||, the numerator estimated through the count sketch of the whole array."""
+        assert tuple(_np(x).shape) == self.shape, f"shape {tuple(_np(x).shape)} vs {self.shape}"
+        d = (sketch(x) - self.sketch).norm().item()
+        if self.norm == 0.0:
+            return 0.0 if _flat64(x).abs().max().item() == 0.0 else float("inf")
+        return d / self.norm
+
+    def sq_dist(self, x) -> float:
+        """||x - ref||^2 estimated through the count sketch (for 0/1 flags: the number of differing elements)."""
+        assert tuple(_np(x).shape) == self.shape, f"shape {tuple(_np(x).shape)} vs {self.shape}"
+        return (sketch(x) - self.sketch).norm().item() ** 2
+
+    def max_err(self, x) -> float:
+        """max |x - ref| / max|ref| over the seeded sample positions."""
+        v = _flat64(x)
+        if self.numel == 0 or self.absmax == 0.0:
+            return 0.0
+        pos = _hash(v.numel(), v.device)[2].to(v.device)
+        return (v[pos].cpu() - self.sample).abs().max().item() / self.absmax
+
+
+def load_golden(name: str) -> dict:
+    d = np.load(os.path.join(GOLDEN_DIR, name))
+    return {str(k): Ref(tuple(int(s) for s in str(sh).split(",") if s), d["digests"][i].tobytes(), d["rows"][i])
+            for i, (k, sh) in enumerate(zip(d["keys"], d["shapes"]))}
+
+
 def make_inputs(scene_kind: str, n: int, W: int, H: int, mode: str, cam_k: int = 0, seed: int = 0,
                 opacity_mode: str = "random", device=None, **cam_kw):
     if scene_kind == "strands":
