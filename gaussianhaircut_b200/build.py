@@ -44,20 +44,15 @@ def needs_build() -> bool:
     return os.path.getmtime(LIB_PATH) < max(os.path.getmtime(p) for p in deps)
 
 
-def build(force: bool = False, verbose: bool = True, extra_flags: list[str] | None = None, variant: str | None = None) -> str:
-    """`variant`: build lib/libgh_raster_<variant>.so with `extra_flags` (-D tunables) next to the product library --
-    used by tools/bench_variants.py to measure kernel variants in one GPU session; the product loads only LIB_PATH."""
-    lib_path = LIB_PATH if variant is None else os.path.join(LIB_DIR, f"libgh_raster_{variant}.so")
-    obj_dir = OBJ_DIR if variant is None else os.path.join(LIB_DIR, f"obj_{variant}")
-    if variant is None and not force and not needs_build():
+def build(force: bool = False, verbose: bool = True) -> str:
+    if not force and not needs_build():
         return LIB_PATH
-    os.makedirs(obj_dir, exist_ok=True)
+    os.makedirs(OBJ_DIR, exist_ok=True)
     nvcc = _nvcc()
-    flags = NVCC_FLAGS + (extra_flags or [])
 
     def compile_one(src: str) -> str:
-        obj = os.path.join(obj_dir, src + ".o")
-        cmd = [nvcc, "-c", os.path.join(CSRC, src), "-o", obj, f"-I{INCLUDE}", f"-I{CSRC}"] + flags
+        obj = os.path.join(OBJ_DIR, src + ".o")
+        cmd = [nvcc, "-c", os.path.join(CSRC, src), "-o", obj, f"-I{INCLUDE}", f"-I{CSRC}"] + NVCC_FLAGS
         if verbose:
             print("[gh build]", " ".join(cmd), flush=True)
         subprocess.run(cmd, check=True)
@@ -65,12 +60,12 @@ def build(force: bool = False, verbose: bool = True, extra_flags: list[str] | No
 
     with ThreadPoolExecutor(max_workers=len(SOURCES)) as ex:
         objs = list(ex.map(compile_one, SOURCES))
-    cmd = [nvcc, "-shared", "-o", lib_path] + objs + ["-gencode", "arch=compute_100a,code=sm_100a",
+    cmd = [nvcc, "-shared", "-o", LIB_PATH] + objs + ["-gencode", "arch=compute_100a,code=sm_100a",
                                                        "-cudart", "static", "-Xcompiler", "-fPIC"]
     if verbose:
         print("[gh build]", " ".join(cmd), flush=True)
     subprocess.run(cmd, check=True)
-    return lib_path
+    return LIB_PATH
 
 
 if __name__ == "__main__":

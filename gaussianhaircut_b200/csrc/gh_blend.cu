@@ -16,47 +16,32 @@
 //     pixel, and every lane walks only ITS pixel's list -- a skipped Gaussian costs nothing;
 //   * the 10 colour channels are accumulated as 5 x (FMUL2 + FFMA2), bit-identical to FMUL + FFMA.
 //   backward (gh_blend_backward_kernel, CTA = tile, 4 warps, a vertical pixel pair per lane)
-//   * one 512-record window staged at a time; Gaussians are scan-converted against the tile's 32 blocks
-//     of 4x2 pixels and a shuffle transpose leaves one bit list per block;
-//   * a block is owned by 4 lanes; the 8 blocks of a warp walk their own lists in lock-step (one warp
-//     instruction works on EIGHT different Gaussians); blocks are assigned to warps by list length;
+//   * one 384-record window staged at a time; Gaussians are scan-converted against the tile's 64 blocks
+//     of 2x2 pixels and two shuffle transposes leave one bit list per block;
+//   * a block is owned by 2 lanes; the 16 blocks of a warp walk their own lists in lock-step (one warp
+//     instruction works on SIXTEEN different Gaussians); blocks are assigned to warps by list length;
 //   * the pixel pair is evaluated in packed FP32 (.x upper pixel, .y lower pixel); the 16 gradient
-//     components are summed over the block's 4 lanes through shared memory and leave as ONE
+//     components are summed over the block's 2 lanes through shared memory and leave as TWO
 //     REDG.E.ADD.F32x4 per lane into a 64-byte per-Gaussian record -- instead of 16 scalar atomicAdd
 //     per (pixel, Gaussian) pair in the reference (backward.cu:527,549-558);
 //   * dL/dalpha uses the scalar form of the reference's per-channel suffix recursion
 //     (backward.cu:519-523):  sum_ch (c - accum_rec)[ch] dL[ch]  =  c.dL  -  A,   A' = a_last (c_last.dL) + (1-a_last) A.
+// Both kernels take tiles by decreasing list length (gh_tile_scan_kernel's permutation `tile_perm`).
+// DESIGN.md section 5 records the alternatives to these choices that were measured and rejected.
 #include "gh_common.cuh"
 #include "gh_kernels.h"
 
 #define GH_HALF_C (GH_NUM_CHANNELS / 2)
 
-// ---- build-time tunables (defaults = the measured best; tools/bench_variants.py rebuilds with -D overrides)
-#ifndef GH_TILE_ORDER
-#define GH_TILE_ORDER 1          // 1: blend CTAs take tiles by decreasing list length (gh_tile_scan_kernel's permutation)
-#endif
-#ifndef GH_FWD_NBUF
-#define GH_FWD_NBUF 2            // forward staging: 2 = double-buffered chunks, 1 = one single-buffered window (other CTAs cover the gather)
-#endif
-#ifndef GH_CHUNK
-#define GH_CHUNK 256             // forward staging chunk / window (records); 512 with GH_FWD_NBUF 1 keeps the same shared memory
-#endif
-#ifndef GH_BWD_CHUNK
+#define GH_CHUNK 256             // forward staging chunk (records): one per thread, two chunks in flight
+#define GH_FWD_MIN_CTAS 4        // __launch_bounds__ second argument of the forward kernel (register cap)
+#define GH_BWD_THREADS 128
 #define GH_BWD_CHUNK 384         // backward staging window (records)
-#endif
-#ifndef GH_BWD_MIN_CTAS
 #define GH_BWD_MIN_CTAS 5        // __launch_bounds__ second argument of the backward kernel (register cap)
-#endif
-#ifndef GH_BWD_LPB
-#define GH_BWD_LPB 2             // lanes per backward block: 4 = 4x2-pixel blocks (8 per warp), 2 = 2x2-pixel blocks (16 per warp)
-#endif
-#define GH_BWD_NBLK (128 / GH_BWD_LPB)          // blocks per tile
-#define GH_BWD_BPW (32 / GH_BWD_LPB)            // blocks per warp
-#define GH_BWD_BW GH_BWD_LPB                    // block width in pixels (a lane owns a vertical pixel pair)
-#define GH_BWD_NBX (16 / GH_BWD_BW)             // blocks across the tile
-#ifndef GH_BWD_FAST_EXP
-#define GH_BWD_FAST_EXP 0        // 1: ex2.approx based exp in the backward (gradients only; decisions may differ in the last ulp)
-#endif
+#define GH_BWD_BLOCKS 64         // backward 2x2-pixel blocks per tile: 8 across, 8 down, 16 per warp
+
+static_assert(GH_CHUNK == 256, "each of the forward kernel's 256 threads stages exactly one record per chunk");
+static_assert(GH_BWD_CHUNK % GH_BWD_THREADS == 0, "every backward thread stages the same number of records of a full window");
 
 namespace {
 
@@ -105,14 +90,15 @@ __device__ __forceinline__ float gh_rcp_approx(float x) {
     return r;
 }
 
+// forward staging, double buffered: chunk c sits in buffer c & 1, chunk c + 1 lands in the other while c is blended
 struct GhStage {
-    float4 g0[GH_FWD_NBUF][GH_CHUNK];
-    float4 g1[GH_FWD_NBUF][GH_CHUNK];
-    float2 feat[GH_FWD_NBUF][GH_CHUNK * GH_HALF_C];
-    uint32_t id[GH_FWD_NBUF][GH_CHUNK];
+    float4 g0[2][GH_CHUNK];
+    float4 g1[2][GH_CHUNK];
+    float2 feat[2][GH_CHUNK * GH_HALF_C];
+    uint32_t id[2][GH_CHUNK];
 };
-static_assert(sizeof(float4) * 2 * GH_FWD_NBUF * GH_CHUNK >= 8u * GH_INKERNEL_SORT_MAX, "sort buffer A (g0+g1) too small");
-static_assert(sizeof(float2) * GH_FWD_NBUF * GH_CHUNK * GH_HALF_C >= 8u * GH_INKERNEL_SORT_MAX, "sort buffer B (feat) too small");
+static_assert(sizeof(GhStage::g0) + sizeof(GhStage::g1) >= 8u * GH_INKERNEL_SORT_MAX, "sort buffer A (g0+g1) too small");
+static_assert(sizeof(GhStage::feat) >= 8u * GH_INKERNEL_SORT_MAX, "sort buffer B (feat) too small");
 
 // issue the gather of one instance (geometry record + feature row) into slot `slot` of buffer `buf`
 __device__ __forceinline__ void gh_stage_issue(GhStage& st, int buf, int slot, uint32_t id,
@@ -213,9 +199,6 @@ __device__ __forceinline__ void gh_build_pixel_lists(const GhStage& st, uint32_t
 }
 
 // ------------------------------------------------------------------------------------------ forward
-#ifndef GH_FWD_MIN_CTAS
-#define GH_FWD_MIN_CTAS 4        // __launch_bounds__ second argument of the forward kernel (register cap)
-#endif
 __global__ void __launch_bounds__(256, GH_FWD_MIN_CTAS)
 gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __restrict__ tile_perm, uint64_t* inst,
                         const GhGeo* __restrict__ geo, const float* __restrict__ features,
@@ -230,7 +213,7 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
     GhStage& st = *reinterpret_cast<GhStage*>(gh_fwd_smem);
     uint32_t* pixbits = reinterpret_cast<uint32_t*>(gh_fwd_smem + sizeof(GhStage));   // [word][pixel] (GH_CHUNK / 32 words x 256); also the sort's scratch
 
-    const int tile = GH_TILE_ORDER ? (int)tile_perm[blockIdx.x] : (int)blockIdx.x;      // heaviest tiles first
+    const int tile = (int)tile_perm[blockIdx.x];      // heaviest tiles first
     const int tx = tile % gx, ty = tile / gx;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     // a warp owns two pixel rows: lanes 0..15 row 2*warp, lanes 16..31 row 2*warp+1
@@ -257,19 +240,7 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
     // one kernel the two overlap across the CTAs of an SM.  The sorted bucket is written back for the
     // backward pass.  Longer lists were sorted by gh_tile_split_long_kernel + gh_segment_sort_kernel
     // (gh_binning.cu) before this launch.
-#ifndef GH_ABLATE_SORT     // (timing experiments only: tools/bench_variants.py)
-#define GH_ABLATE_SORT 0
-#endif
-#ifndef GH_ABLATE_TRAVERSE
-#define GH_ABLATE_TRAVERSE 0
-#endif
-#ifndef GH_ABLATE_BUILD
-#define GH_ABLATE_BUILD 0
-#endif
-#ifndef GH_ABLATE_GATHER
-#define GH_ABLATE_GATHER 0
-#endif
-    if (!GH_ABLATE_SORT && n >= 2 && n <= (int)GH_INKERNEL_SORT_MAX) {
+    if (n >= 2 && n <= (int)GH_INKERNEL_SORT_MAX) {
         uint64_t* sbase = reinterpret_cast<uint64_t*>(&st.g0[0][0]);     // g0 + g1 = 16 KB contiguous
         uint64_t* spong = reinterpret_cast<uint64_t*>(&st.feat[0][0]);   // next 16 KB (feat is 20 KB)
         uint64_t* gl = inst + rg.x;
@@ -310,63 +281,36 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
         __syncthreads();
     }
 
-#if GH_FWD_NBUF == 2
     // prologue: chunk 0 in flight, indices of chunk 1 in a register
     uint32_t next_id = 0;
     if (nchunks > 0) {
-        if (!GH_ABLATE_GATHER && tid < min(GH_CHUNK, n)) gh_stage_issue(st, 0, tid, (uint32_t)inst[(size_t)rg.x + tid], geo, features);
+        if (tid < min(GH_CHUNK, n)) gh_stage_issue(st, 0, tid, (uint32_t)inst[(size_t)rg.x + tid], geo, features);
         gh_cp_async_commit();
         if (GH_CHUNK + tid < n) next_id = (uint32_t)inst[(size_t)rg.x + GH_CHUNK + tid];
     }
-#else
-    constexpr int PER_THREAD = GH_CHUNK / 256;
-    uint32_t next_id[PER_THREAD];
-#pragma unroll
-    for (int h = 0; h < PER_THREAD; h++) next_id[h] = (tid + h * 256 < n) ? (uint32_t)inst[(size_t)rg.x + tid + h * 256] : 0u;
-#endif
 
     for (int c = 0; c < nchunks; c++) {
         const int base = c * GH_CHUNK;
         const int cnt = min(GH_CHUNK, n - base);
-#if GH_FWD_NBUF == 2
         const int buf = c & 1;
         gh_cp_async_wait_all();
         // chunk c landed for every thread; block-wide early exit like the reference's
         // __syncthreads_count(done) == BLOCK_SIZE
         if (__syncthreads_and(warp_done)) break;
         if (c + 1 < nchunks) {
-            if (!GH_ABLATE_GATHER && base + GH_CHUNK + tid < n) gh_stage_issue(st, buf ^ 1, tid, next_id, geo, features);
+            if (base + GH_CHUNK + tid < n) gh_stage_issue(st, buf ^ 1, tid, next_id, geo, features);
             gh_cp_async_commit();
             if (base + 2 * GH_CHUNK + tid < n) next_id = (uint32_t)inst[(size_t)rg.x + base + 2 * GH_CHUNK + tid];
         }
-        if (!GH_ABLATE_BUILD) gh_build_pixel_lists(st, pixbits, buf, cnt, warp, lane, tx0, ty0);
+        gh_build_pixel_lists(st, pixbits, buf, cnt, warp, lane, tx0, ty0);
         __syncthreads();
-#else
-        constexpr int buf = 0;
-        // everyone is done with the previous window; block-wide early exit like the reference's
-        // __syncthreads_count(done) == BLOCK_SIZE
-        if (__syncthreads_and(warp_done)) break;
-#pragma unroll
-        for (int h = 0; h < PER_THREAD; h++)
-            if (tid + h * 256 < cnt) gh_stage_issue(st, 0, tid + h * 256, next_id[h], geo, features);
-        gh_cp_async_commit();
-#pragma unroll
-        for (int h = 0; h < PER_THREAD; h++) {
-            const int nx = base + GH_CHUNK + tid + h * 256;
-            next_id[h] = (nx < n) ? (uint32_t)inst[(size_t)rg.x + nx] : 0u;
-        }
-        gh_cp_async_wait_all();
-        __syncthreads();
-        for (int word = warp; word * 32 < cnt; word += 8) gh_build_pixel_lists(st, pixbits, 0, cnt, word, lane, tx0, ty0);
-        __syncthreads();
-#endif
 
-        if (!done && !GH_ABLATE_TRAVERSE) {
+        if (!done) {
             // which of my pixel's 8 list words are non-empty
             uint32_t nz = 0u;
 #pragma unroll
             for (int k = 0; k < GH_CHUNK / 32; k++)
-                if (GH_FWD_NBUF == 2 || k * 32 < cnt) nz |= (pixbits[k * 256 + tid] != 0u) ? (1u << k) : 0u;
+                nz |= (pixbits[k * 256 + tid] != 0u) ? (1u << k) : 0u;
             int wi = 0;
             uint32_t cur = 0u;
             while (true) {
@@ -413,15 +357,15 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
 
 // ------------------------------------------------------------------------------------------ backward
 // Backward staging: ONE window of GH_BWD_CHUNK instances (single-buffered; the other resident CTAs of
-// the SM cover the gather latency).  The 8 blocks of a warp walk their lists in lock-step, so a warp
-// spends max(list length over its blocks) steps per window: a 512-wide window wastes fewer lanes on
-// that maximum than two 256-wide ones (tools/imbalance.py: 0.74 vs 0.69 lane efficiency at 500k).
+// the SM cover the gather latency).  The 16 blocks of a warp walk their lists in lock-step, so a warp
+// spends max(list length over its blocks) steps per window: a wide window wastes fewer lanes on that
+// maximum than several narrow ones (tools/imbalance.py), and 384 records still leave room for 5 CTAs per SM.
 struct GhStageB {
     float4 g0[GH_BWD_CHUNK];
     float4 g1[GH_BWD_CHUNK];
     float2 feat[GH_BWD_CHUNK * GH_HALF_C];
     uint32_t id[GH_BWD_CHUNK];
-    uint32_t bits[GH_BWD_NBLK][GH_BWD_CHUNK / 32 + 1];   // [block][word]; +1 pad against bank conflicts
+    uint32_t bits[GH_BWD_BLOCKS][GH_BWD_CHUNK / 32 + 1];   // [block][word]; +1 pad against bank conflicts
 };
 
 __device__ __forceinline__ void gh_stage_issue_b(GhStageB& st, int slot, uint32_t id,
@@ -435,49 +379,14 @@ __device__ __forceinline__ void gh_stage_issue_b(GhStageB& st, int slot, uint32_
     st.id[slot] = id;
 }
 
-// Which of the tile's 32 blocks (4 wide x 2 high; bit = by*4 + bx) can this Gaussian reach with
-// alpha >= 1/255?  Exact-conservative: on each pixel row the set {q(d) <= 2(thr+slack)} is an
-// x-interval obtained from the quadratic; the interval is widened by 0.01 px and rounded outwards to
-// whole pixels.  Returns all ones when the conic is not positive definite (no bound available).
-// Skipping a Gaussian in a block whose bit is clear cannot change any pixel of that block: each of
-// them would take the reference's `alpha < 1/255 -> continue` (forward.cu:370, backward.cu:503).
-// Two pixel rows per instruction; a row without a real span has disc <= 0 -> s = NaN -> fminf / fmaxf
-// ignore it.
-#if GH_BWD_LPB == 4      // (the 4x2-block variant of the measured A/B, DESIGN.md section 5; the product builds 2x2)
-__device__ __forceinline__ uint32_t gh_block_mask2(const float4 g0, const float4 g1, float tx0, float ty0) {
-    const float gx = g0.x, gy = g0.y, a = g0.z, b = g0.w, c = g1.x, thr = g1.z, pd = g1.w;
-    if (pd == 0.f) return 0xffffffffu;
-    const float mxd = fmaxf(fabsf(gx - tx0), fabsf(gx - (tx0 + 15.f)));
-    const float myd = fmaxf(fabsf(gy - ty0), fabsf(gy - (ty0 + 15.f)));
-    const float slack = 1e-3f + 2e-5f * (a * mxd * mxd + c * myd * myd + 2.f * fabsf(b) * mxd * myd);
-    const float Q = 2.f * (thr + slack);
-    if (!(Q >= 0.f)) return (Q != Q) ? 0xffffffffu : 0u;
-    const float2 ia = gh_f2(__frcp_rn(a)), aQ = gh_f2(a * Q), bbac = gh_f2(b * b - a * c), gx2 = gh_f2(gx), b2 = gh_f2(b);
-    float2 dy = make_float2(gy - ty0, gy - (ty0 + 1.f));     // rows 2 by, 2 by + 1
-    uint32_t mask = 0;
-#pragma unroll
-    for (int by = 0; by < 8; by++) {
-        // a dx^2 + 2 b dy dx + (c dy^2 - Q) <= 0,  dx = gx - px
-        const float2 disc = gh_fma2(gh_mul2(dy, dy), bbac, aQ);
-        const float2 s = gh_mul2(disc, make_float2(rsqrtf(disc.x), rsqrtf(disc.y)));   // NaN unless disc > 0
-        const float2 hb = gh_mul2(b2, dy);
-        const float2 lo2 = gh_fma2(gh_sub2(hb, s), ia, gx2), hi2 = gh_fma2(gh_add2(hb, s), ia, gx2);
-        const float xlo = fminf(fminf(1e30f, lo2.x), lo2.y), xhi = fmaxf(fmaxf(-1e30f, hi2.x), hi2.y);
-        // tile-local integer pixel columns inside [xlo - .01, xhi + .01]
-        const float lo = (xlo - 0.01f) - tx0, hi = (xhi + 0.01f) - tx0;
-        const int p0 = max(0, __float2int_ru(lo)), p1 = min(15, __float2int_rd(hi));
-        if (p0 <= p1) {
-            const int b0 = p0 >> 2, b1 = p1 >> 2;
-            mask |= (((2u << (b1 - b0)) - 1u) << b0) << (4 * by);
-        }
-        dy = gh_add2(dy, gh_f2(-2.f));
-    }
-    return mask;
-}
-#endif
-
-// The same test at 2x2-block granularity: 64 blocks, bit = by * 8 + bx; .x = block rows 0..3, .y = rows 4..7.
-#if GH_BWD_LPB != 4
+// Which of the tile's 64 blocks (2x2 pixels; bit = by * 8 + bx, .x = block rows 0..3, .y = rows 4..7)
+// can this Gaussian reach with alpha >= 1/255?  Exact-conservative: on each pixel row the set
+// {q(d) <= 2(thr+slack)} is an x-interval obtained from the quadratic; the interval is widened by
+// 0.01 px and rounded outwards to whole pixels.  Returns all ones when the conic is not positive
+// definite (no bound available).  Skipping a Gaussian in a block whose bit is clear cannot change any
+// pixel of that block: each of them would take the reference's `alpha < 1/255 -> continue`
+// (forward.cu:370, backward.cu:503).  Two pixel rows (one block row) per instruction; a row without a
+// real span has disc <= 0 -> s = NaN -> fminf / fmaxf ignore it.
 __device__ __forceinline__ uint2 gh_block_mask_2x2(const float4 g0, const float4 g1, float tx0, float ty0) {
     const float gx = g0.x, gy = g0.y, a = g0.z, b = g0.w, c = g1.x, thr = g1.z, pd = g1.w;
     if (pd == 0.f) return make_uint2(0xffffffffu, 0xffffffffu);
@@ -491,11 +400,13 @@ __device__ __forceinline__ uint2 gh_block_mask_2x2(const float4 g0, const float4
     uint32_t m[2] = {0u, 0u};
 #pragma unroll
     for (int by = 0; by < 8; by++) {
+        // a dx^2 + 2 b dy dx + (c dy^2 - Q) <= 0,  dx = gx - px
         const float2 disc = gh_fma2(gh_mul2(dy, dy), bbac, aQ);
         const float2 s = gh_mul2(disc, make_float2(rsqrtf(disc.x), rsqrtf(disc.y)));   // NaN unless disc > 0
         const float2 hb = gh_mul2(b2, dy);
         const float2 lo2 = gh_fma2(gh_sub2(hb, s), ia, gx2), hi2 = gh_fma2(gh_add2(hb, s), ia, gx2);
         const float xlo = fminf(fminf(1e30f, lo2.x), lo2.y), xhi = fmaxf(fmaxf(-1e30f, hi2.x), hi2.y);
+        // tile-local integer pixel columns inside [xlo - .01, xhi + .01]
         const float lo = (xlo - 0.01f) - tx0, hi = (xhi + 0.01f) - tx0;
         const int p0 = max(0, __float2int_ru(lo)), p1 = min(15, __float2int_rd(hi));
         if (p0 <= p1) {
@@ -506,28 +417,20 @@ __device__ __forceinline__ uint2 gh_block_mask_2x2(const float4 g0, const float4
     }
     return make_uint2(m[0], m[1]);
 }
-#endif
 
-// batch `word` = instances [32 word, 32 word + 32) of the window, one per lane; a 5-step shuffle
-// transpose turns the 32 block masks into one list word per block (lane = block).  The word is cut at
-// the block's deepest blended list position `glast` here, once, rather than in the traversal loop.
+// batch `word` = instances [32 word, 32 word + 32) of the window, one per lane; two 5-step shuffle
+// transposes turn the 32 block masks into one list word per block (lane = block `lane` and block
+// 32 + lane).  The word is cut at the block's deepest blended list position `glast` here, once, rather
+// than in the traversal loop.
 __device__ __forceinline__ uint32_t gh_valid_bits(uint32_t glast, int first_pos) {
     const int lim = (int)glast - first_pos;
     return lim >= 32 ? 0xffffffffu : (lim <= 0 ? 0u : ((1u << lim) - 1u));
 }
 
-// glast_lo / glast_hi: deepest blended list position of block `lane` (and, with 64 blocks, of block 32 + lane)
+// glast_lo / glast_hi: deepest blended list position of block `lane` / of block 32 + lane
 __device__ __forceinline__ void gh_build_lists_b(GhStageB& st, int cnt, int word, int lane, float tx0, float ty0,
                                                  int base, uint32_t glast_lo, uint32_t glast_hi) {
     const int j = word * 32 + lane;
-#if GH_BWD_LPB == 4
-    uint32_t m = 0;
-    if (j < cnt) m = gh_block_mask2(st.g0[j], st.g1[j], tx0, ty0);
-    uint32_t mine = 0;
-    if (__any_sync(0xffffffffu, m != 0u)) mine = gh_transpose32(m, lane);
-    st.bits[lane][word] = mine & gh_valid_bits(glast_lo, base + word * 32);
-    (void)glast_hi;
-#else
     uint2 m = make_uint2(0u, 0u);
     if (j < cnt) m = gh_block_mask_2x2(st.g0[j], st.g1[j], tx0, ty0);
     uint32_t lo = 0, hi = 0;
@@ -535,46 +438,17 @@ __device__ __forceinline__ void gh_build_lists_b(GhStageB& st, int cnt, int word
     if (__any_sync(0xffffffffu, m.y != 0u)) hi = gh_transpose32(m.y, lane);
     st.bits[lane][word] = lo & gh_valid_bits(glast_lo, base + word * 32);
     st.bits[32 + lane][word] = hi & gh_valid_bits(glast_hi, base + word * 32);
-#endif
 }
 
-// CTA = tile = 4 warps.  A lane owns a vertical pixel pair (x, y0), (x, y0+1); 4 lanes own a 4x2 block;
-// the 8 blocks of a warp walk their own lists in lock-step, i.e. every warp instruction works on EIGHT
-// different Gaussians.  The two pixels of a lane are summed in registers; the 16 gradient components
-// are then summed over the 4 lanes through shared memory (gh_group4_reduce16), leaving four adjacent
-// components per lane = one REDG.E.ADD.F32x4 per lane.
-#define GH_BWD_THREADS 128
+// Per-lane record of the reduction buffer, in float4.  gh_group2_reduce16 uses 3 of the 5 (the buffer
+// still has the size of an earlier 4-lane reduction; shrinking it changes the launch's shared memory).
+#define GH_RED_STRIDE4 5
 
-// Sum the 16 gradient components over the 4 lanes of a block and leave components 4*(lane&3)+{0..3}
-// in each lane.  Through shared memory: 4 STS.128 + 4 LDS.128 + 6 FADD2 per lane, against 12 SHFL +
-// 24 SEL + 6 FADD2 for a transposing butterfly (the kernel is bound by issue slots).  A lane's record
-// is 80 B (16 floats + pad): the 8 lanes of a quarter-warp store to, and load from, 8 disjoint groups
-// of 4 banks.
-#define GH_RED_STRIDE4 5       // float4 per lane record
-#if GH_BWD_LPB == 4
-__device__ __forceinline__ float4 gh_group4_reduce16(const float (&v)[16], float4* warp_buf, int lane) {
-    float4* mine = warp_buf + lane * GH_RED_STRIDE4;
-    mine[0] = make_float4(v[0], v[1], v[2], v[3]);
-    mine[1] = make_float4(v[4], v[5], v[6], v[7]);
-    mine[2] = make_float4(v[8], v[9], v[10], v[11]);
-    mine[3] = make_float4(v[12], v[13], v[14], v[15]);
-    __syncwarp();
-    const float4* grp = warp_buf + (lane & 28) * GH_RED_STRIDE4 + (lane & 3);
-    const float4 a = grp[0], b = grp[GH_RED_STRIDE4], c = grp[2 * GH_RED_STRIDE4], d = grp[3 * GH_RED_STRIDE4];
-    __syncwarp();              // the next step overwrites the records
-    const float2 lo = gh_add2(gh_add2(make_float2(a.x, a.y), make_float2(b.x, b.y)),
-                              gh_add2(make_float2(c.x, c.y), make_float2(d.x, d.y)));
-    const float2 hi = gh_add2(gh_add2(make_float2(a.z, a.w), make_float2(b.z, b.w)),
-                              gh_add2(make_float2(c.z, c.w), make_float2(d.z, d.w)));
-    return make_float4(lo.x, lo.y, hi.x, hi.y);
-}
-#endif
-
-// 2-lane blocks: the even lane keeps components 0..7, the odd lane 8..15 (two REDG.E.ADD.F32x4 each).  Each lane
+// The even lane keeps components 0..7, the odd lane 8..15 (two REDG.E.ADD.F32x4 each).  Each lane
 // stores the half its partner keeps (2 STS.128), loads the partner's contribution to its own half (2 LDS.128) and
-// adds (4 FADD2).  Record stride 48 B: the 8 lanes of a quarter-warp hit 8 disjoint groups of 4 banks.
+// adds (4 FADD2): 4 shared-memory instructions where a shuffle exchange of 8 floats takes 8 SHFL (the kernel is
+// bound by issue slots).  Record stride 48 B: the 8 lanes of a quarter-warp hit 8 disjoint groups of 4 banks.
 #define GH_RED2_STRIDE4 3
-#if GH_BWD_LPB != 4
 __device__ __forceinline__ void gh_group2_reduce16(const float (&v)[16], float4* warp_buf, int lane, float4& out0, float4& out1) {
     const bool odd = (lane & 1) != 0;
     float4* mine = warp_buf + lane * GH_RED2_STRIDE4;
@@ -592,7 +466,6 @@ __device__ __forceinline__ void gh_group2_reduce16(const float (&v)[16], float4*
     out0 = make_float4(s0.x, s0.y, s1.x, s1.y);
     out1 = make_float4(s2.x, s2.y, s3.x, s3.y);
 }
-#endif
 
 // State of the lane's pixel pair; .x = pixel (x, y0), .y = pixel (x, y0 + 1).
 struct GhBwdPair {
@@ -619,13 +492,8 @@ __device__ __forceinline__ bool gh_bwd_pair(GhBwdPair& p, const float4 g0, const
     const float2 t3 = gh_mul2(dy, gh_mul2(dy, gh_f2(g1.x)));
     const float2 sq = gh_fma2(dx2, gh_f2(t1), t3);
     const float2 power = gh_fma2(sq, gh_f2(-0.5f), gh_mul2(dy, gh_f2(-dxcb)));
-#if GH_BWD_FAST_EXP
-    const float Gx0 = __expf((power.x > 0.0f) ? 0.0f : power.x);
-    const float Gx1 = __expf((power.y > 0.0f) ? 0.0f : power.y);
-#else
     const float Gx0 = expf((power.x > 0.0f) ? 0.0f : power.x);   // expf(power) whenever the reference evaluates it
     const float Gx1 = expf((power.y > 0.0f) ? 0.0f : power.y);
-#endif
     const float2 ao = gh_mul2(gh_f2(g1.y), make_float2(Gx0, Gx1));
     const float alpha0 = fminf(0.99f, ao.x), alpha1 = fminf(0.99f, ao.y);
     const bool ok0 = (pos < p.last0) & !(power.x > 0.0f) & !(alpha0 < 1.0f / 255.0f);
@@ -675,6 +543,12 @@ __device__ __forceinline__ bool gh_bwd_pair(GhBwdPair& p, const float4 g0, const
     return ok0 | ok1;
 }
 
+// CTA = tile = 4 warps.  A lane owns a vertical pixel pair (x, y0), (x, y0+1); lanes 2i and 2i+1 own a 2x2
+// block; block b covers tile pixels x = 2 (b % 8) + {0, 1}, y = 2 (b / 8) + {0, 1}.  The 16 blocks of a warp
+// walk their own lists in lock-step, i.e. every warp instruction works on SIXTEEN different Gaussians.  The
+// two pixels of a lane are summed in registers; the 16 gradient components are then summed over the block's
+// 2 lanes through shared memory (gh_group2_reduce16), leaving eight adjacent components per lane = two
+// REDG.E.ADD.F32x4 per lane.
 __global__ void __launch_bounds__(GH_BWD_THREADS, GH_BWD_MIN_CTAS)
 gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __restrict__ tile_perm, const uint64_t* __restrict__ inst,
                          const GhGeo* __restrict__ geo, const float* __restrict__ features,
@@ -687,32 +561,30 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
     GhStageB& st = *reinterpret_cast<GhStageB*>(gh_bwd_smem);
     float4* red_buf = reinterpret_cast<float4*>(gh_bwd_smem + sizeof(GhStageB)) + (threadIdx.x >> 5) * 32 * GH_RED_STRIDE4;
     __shared__ uint32_t s_warp_last[GH_BWD_THREADS / 32];
-    __shared__ uint32_t s_glast[GH_BWD_NBLK];              // per block: deepest list position any of its pixels blended
-    __shared__ uint8_t s_perm[GH_BWD_THREADS / 32][GH_BWD_NBLK];   // per warp (redundant copies): rank -> block
+    __shared__ uint32_t s_glast[GH_BWD_BLOCKS];              // per block: deepest list position any of its pixels blended
+    __shared__ uint8_t s_perm[GH_BWD_THREADS / 32][GH_BWD_BLOCKS];   // per warp (redundant copies): rank -> block
 
-    const int tile = GH_TILE_ORDER ? (int)tile_perm[blockIdx.x] : (int)blockIdx.x;      // heaviest tiles first
+    const int tile = (int)tile_perm[blockIdx.x];      // heaviest tiles first
     const int tx = tile % gx, ty = tile / gx;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const float tx0 = (float)(tx * GH_BLOCK_X), ty0 = (float)(ty * GH_BLOCK_Y);
-    const unsigned gshift = lane & (32 - GH_BWD_LPB);      // first lane of my block
-    const unsigned gmask = (1u << GH_BWD_LPB) - 1u;
     const size_t plane = (size_t)H * W;
     const uint2 rg = ranges[tile];
 
-    // ---- how far do the blocks / the tile reach into the list?  (natural block order here)
+    // ---- how far do the blocks / the tile reach into the list?  (natural block order here: warp w owns
+    // blocks 16 w .. 16 w + 15)
     {
-        const int nb = GH_BWD_BPW * warp + lane / GH_BWD_LPB;
-        const int nx = tx * GH_BLOCK_X + GH_BWD_BW * (nb % GH_BWD_NBX) + (lane % GH_BWD_LPB);
-        const int ny = ty * GH_BLOCK_Y + 2 * (nb / GH_BWD_NBX);
+        const int nb = 16 * warp + lane / 2;
+        const int nx = tx * GH_BLOCK_X + 2 * (nb % 8) + (lane % 2);
+        const int ny = ty * GH_BLOCK_Y + 2 * (nb / 8);
         uint32_t gl = 0;
         if (nx < W && ny < H) gl = n_contrib[(size_t)ny * W + nx];
         if (nx < W && ny + 1 < H) gl = max(gl, n_contrib[(size_t)(ny + 1) * W + nx]);
-#pragma unroll
-        for (int o = GH_BWD_LPB / 2; o > 0; o >>= 1) gl = max(gl, __shfl_xor_sync(0xffffffffu, gl, o));
-        if ((lane % GH_BWD_LPB) == 0) s_glast[nb] = gl;
+        gl = max(gl, __shfl_xor_sync(0xffffffffu, gl, 1));      // over the block's two lanes
+        if ((lane % 2) == 0) s_glast[nb] = gl;
         uint32_t wl = gl;
 #pragma unroll
-        for (int o = GH_BWD_LPB; o < 32; o <<= 1) wl = max(wl, __shfl_xor_sync(0xffffffffu, wl, o));
+        for (int o = 2; o < 32; o <<= 1) wl = max(wl, __shfl_xor_sync(0xffffffffu, wl, o));
         if (lane == 0) s_warp_last[warp] = wl;
     }
     __syncthreads();
@@ -723,9 +595,9 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
     const int nchunks = (n + GH_BWD_CHUNK - 1) / GH_BWD_CHUNK;
     if (nchunks == 0) return;
     constexpr int PER_THREAD = GH_BWD_CHUNK / GH_BWD_THREADS;
-    // the builder's lane == block after the transpose (with 64 blocks: blocks `lane` and `32 + lane`)
+    // the builder's lane == block after the transposes: blocks `lane` and `32 + lane`
     const uint32_t glast_lo = s_glast[lane];
-    const uint32_t glast_hi = (GH_BWD_NBLK > 32) ? s_glast[(32 + lane) % GH_BWD_NBLK] : 0u;
+    const uint32_t glast_hi = s_glast[32 + lane];
 
     // ---- stage the last window (windows are visited last to first) and build its lists
     uint32_t next_id[PER_THREAD];
@@ -752,7 +624,7 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
 
     // ---- block -> (warp, lane group) assignment.  The blocks of a warp advance in lock-step, so a warp pays for
     // its LONGEST list: blocks are ranked by the length of their list in the window just built (lane b counts block
-    // b -- and block 32 + b; every warp computes the same ranking for itself) and each warp takes GH_BWD_BPW
+    // b -- and block 32 + b; every warp computes the same ranking for itself) and each warp takes 16
     // neighbours of that ranking.  Any assignment gives the same gradients up to the order of the float atomics.
     int blk;
     {
@@ -760,27 +632,24 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
         uint32_t len0 = 0, len1 = 0;
         for (int w = 0; w < nw; w++) {
             len0 += __popc(st.bits[lane][w]);
-            if (GH_BWD_NBLK > 32) len1 += __popc(st.bits[(32 + lane) % GH_BWD_NBLK][w]);
+            len1 += __popc(st.bits[32 + lane][w]);
         }
         const uint32_t key0 = (len0 << 6) | (uint32_t)lane, key1 = (len1 << 6) | (uint32_t)(32 + lane);
         int rank0 = 0, rank1 = 0;
 #pragma unroll
         for (int k = 0; k < 32; k++) {
             const uint32_t a = __shfl_sync(0xffffffffu, key0, k);
-            rank0 += (a < key0) ? 1 : 0;
-            if (GH_BWD_NBLK > 32) {
-                const uint32_t b = __shfl_sync(0xffffffffu, key1, k);
-                rank0 += (b < key0) ? 1 : 0;
-                rank1 += ((a < key1) ? 1 : 0) + ((b < key1) ? 1 : 0);
-            }
+            const uint32_t b = __shfl_sync(0xffffffffu, key1, k);
+            rank0 += ((a < key0) ? 1 : 0) + ((b < key0) ? 1 : 0);
+            rank1 += ((a < key1) ? 1 : 0) + ((b < key1) ? 1 : 0);
         }
         s_perm[warp][rank0] = (uint8_t)lane;
-        if (GH_BWD_NBLK > 32) s_perm[warp][rank1] = (uint8_t)(32 + lane);
+        s_perm[warp][rank1] = (uint8_t)(32 + lane);
         __syncwarp();
-        blk = s_perm[warp][GH_BWD_BPW * warp + lane / GH_BWD_LPB];
+        blk = s_perm[warp][16 * warp + lane / 2];
     }
-    const int px = tx * GH_BLOCK_X + GH_BWD_BW * (blk % GH_BWD_NBX) + (lane % GH_BWD_LPB);
-    const int py0 = ty * GH_BLOCK_Y + 2 * (blk / GH_BWD_NBX);
+    const int px = tx * GH_BLOCK_X + 2 * (blk % 8) + (lane % 2);
+    const int py0 = ty * GH_BLOCK_Y + 2 * (blk / 8);
     const float pxf = (float)px;
 
     GhBwdPair pr;
@@ -818,7 +687,7 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
 
     uint32_t wlast = s_glast[blk];
 #pragma unroll
-    for (int o = GH_BWD_LPB; o < 32; o <<= 1) wlast = max(wlast, __shfl_xor_sync(0xffffffffu, wlast, o));
+    for (int o = 2; o < 32; o <<= 1) wlast = max(wlast, __shfl_xor_sync(0xffffffffu, wlast, o));   // over the warp's blocks
 
     for (int c = nchunks - 1; c >= 0; c--) {
         const int base = c * GH_BWD_CHUNK;
@@ -861,21 +730,13 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
             const bool contrib = gh_bwd_pair(pr, g0, g1, feat, pxf, pos, ddelx_dx, ddely_dy, v);
             const uint32_t cm = __ballot_sync(0xffffffffu, contrib);
             if (cm == 0u) continue;
-#if GH_BWD_LPB == 4
-            const float4 s = gh_group4_reduce16(v, red_buf, lane);
-            if ((cm >> gshift) & gmask) {
-                float4* dst = reinterpret_cast<float4*>(acc16 + (size_t)id * 16) + (lane & 3);
-                atomicAdd(dst, s);    // REDG.E.ADD.F32x4
-            }
-#else
             float4 s0, s1;
             gh_group2_reduce16(v, red_buf, lane, s0, s1);
-            if ((cm >> gshift) & gmask) {
+            if ((cm >> (lane & 30)) & 3u) {            // either lane of my block contributed
                 float4* dst = reinterpret_cast<float4*>(acc16 + (size_t)id * 16) + 2 * (lane & 1);
                 atomicAdd(dst, s0);       // REDG.E.ADD.F32x4: components 0..3 / 8..11
                 atomicAdd(dst + 1, s1);   //                              4..7 / 12..15
             }
-#endif
         }
     }
     gh_cp_async_wait_all();

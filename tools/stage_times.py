@@ -1,5 +1,5 @@
-"""Per-stage device times of one library build on the benchmark scene (used by tools/bench_variants.py).
-   python tools/stage_times.py [path/to/libgh_raster_variant.so] [--strands 5000] [--mode native]"""
+"""Per-stage device times of one library build on the benchmark scene; without a path, the in-tree build.
+   python tools/stage_times.py [path/to/libgh_raster.so] [--strands 5000] [--mode native]"""
 import argparse, json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -13,7 +13,7 @@ args = ap.parse_args()
 import torch
 from gaussianhaircut_b200 import _capi
 if args.lib:
-    _capi.LIB_PATH = os.path.abspath(args.lib)      # development only: measure a variant build
+    _capi.LIB_PATH = os.path.abspath(args.lib)      # development only: measure another build of the library
 from gaussianhaircut_b200 import _C
 import synth
 dev = torch.device("cuda:0")
