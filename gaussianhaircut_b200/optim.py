@@ -111,6 +111,8 @@ class FusedAdam:
                         raise RuntimeError(f"FusedAdam: {name} of parameter group '{g.get('name', '?')}' has {t.numel()} "
                                            f"elements ({t.dtype}, {t.device}), the parameter has {n}: optimizer state "
                                            "and parameter went out of sync (densification must replace both)")
+                if n == 0:
+                    continue      # nothing to update, and a tensor without elements has no storage to hand to the kernel
                 ps.append(p); gs.append(gr); ms.append(st["exp_avg"]); vs.append(st["exp_avg_sq"])
                 ns.append(n); lrs.append(float(g["lr"]))
         if not ps:
