@@ -14,10 +14,11 @@
 //     {alpha >= 1/255} on every pixel row (two rows per packed-FP32 instruction) gives 16-bit row masks,
 //     a 5-step shuffle transpose turns the 32 (Gaussian) x 32 (pixel) bit matrix into one hit list per
 //     pixel, and every lane walks only ITS pixel's list -- a skipped Gaussian costs nothing;
-//   * the 10 colour channels are accumulated as 5 x (FMUL2 + FFMA2), bit-identical to FMUL + FFMA.
+//   * the 10 colour channels are accumulated as 5 x (FMUL2 + FFMA2), bit-identical to FMUL + FFMA;
+//   * from the same row masks each record's mask over the backward's 64 blocks of 2x2 pixels is written out.
 //   backward (gh_blend_backward_kernel, CTA = tile, 4 warps, a vertical pixel pair per lane)
-//   * one 384-record window staged at a time; Gaussians are scan-converted against the tile's 64 blocks
-//     of 2x2 pixels and two shuffle transposes leave one bit list per block;
+//   * one 384-position window at a time; only the records whose block mask is not zero are staged, and two
+//     shuffle transposes of their masks leave one bit list per block;
 //   * a block is owned by 2 lanes; the 16 blocks of a warp walk their own lists in lock-step (one warp
 //     instruction works on SIXTEEN different Gaussians); blocks are assigned to warps by list length;
 //   * the pixel pair is evaluated in packed FP32 (.x upper pixel, .y lower pixel); the 16 gradient
@@ -114,7 +115,7 @@ __device__ __forceinline__ void gh_stage_issue(GhStage& st, int buf, int slot, u
 
 // Per-PIXEL instance lists of one staged chunk (forward pass).  Warp w scan-converts Gaussians
 // [32w, 32w+32) of the chunk (one per lane): on every pixel row the exact-conservative x-span of
-// {alpha >= 1/255} (same quadratic as gh_block_mask) becomes a 16-bit column mask; two rows form the
+// {alpha >= 1/255} becomes a 16-bit column mask; two rows form the
 // 32-bit coverage word of the 32 pixels owned by one warp (pixel p = 32*(row/2) + 16*(row%2) + col).
 // The 32 (Gaussian) x 32 (pixel) bit matrix is then transposed inside the warp with 5 shuffle steps,
 // so lane P ends with "which of my warp's 32 Gaussians cover pixel P" and stores it: no atomics, no
@@ -130,8 +131,22 @@ __device__ __forceinline__ uint32_t gh_transpose32(uint32_t x, int lane) {
     return x;
 }
 
+// Two 16-pixel rows (lo, hi halves of `rows`) -> one 8-bit row of 2x2 blocks: bit bx is set when column 2 bx
+// or 2 bx + 1 is set in either row.
+__device__ __forceinline__ uint32_t gh_block_row(uint32_t rows) {
+    uint32_t x = (rows | (rows >> 16)) & 0xffffu;
+    x = (x | (x >> 1)) & 0x5555u;
+    x = (x | (x >> 1)) & 0x3333u;
+    x = (x | (x >> 2)) & 0x0f0fu;
+    return (x | (x >> 4)) & 0x00ffu;
+}
+
+// Besides the pixel lists, every record of the chunk leaves its mask over the backward's 64 blocks of 2x2
+// pixels in bmask[j] (bit by * 8 + bx; .x = block rows 0..3, .y = rows 4..7), derived from the same row
+// masks: the backward stages only the records whose mask is not zero and scan-converts nothing itself.
 __device__ __forceinline__ void gh_build_pixel_lists(const GhStage& st, uint32_t* pixbits, int buf, int cnt,
-                                                     int warp, int lane, float tx0, float ty0) {
+                                                     int warp, int lane, float tx0, float ty0,
+                                                     uint2* __restrict__ bmask) {
     // `warp` = index of the batch of 32 staged Gaussians this warp scan-converts (= list word index)
     const int j = warp * 32 + lane;
     uint32_t rowmask[16];
@@ -189,13 +204,17 @@ __device__ __forceinline__ void gh_build_pixel_lists(const GhStage& st, uint32_t
         rowmask[2 * t] = all_pixels ? 0xffffu : ma;      // rows outside [r0, r1] have disc <= 0
         rowmask[2 * t + 1] = all_pixels ? 0xffffu : mb;
     }
+    uint2 bm = make_uint2(0u, 0u);
 #pragma unroll
     for (int t = 0; t < 8; t++) {
         const uint32_t word = rowmask[2 * t] | (rowmask[2 * t + 1] << 16);   // my coverage of warp t's pixels
+        if (t < 4) bm.x |= gh_block_row(word) << (8 * t);
+        else bm.y |= gh_block_row(word) << (8 * (t - 4));
         uint32_t col = 0u;
         if (__any_sync(0xffffffffu, word != 0u)) col = gh_transpose32(word, lane);
         pixbits[warp * 256 + t * 32 + lane] = col;                           // pixel 32t+lane: bits = Gaussians
     }
+    if (j < cnt) bmask[j] = bm;
 }
 
 // ------------------------------------------------------------------------------------------ forward
@@ -204,7 +223,7 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
                         const GhGeo* __restrict__ geo, const float* __restrict__ features,
                         int W, int H, int gx, const float* __restrict__ bg,
                         float* __restrict__ final_T, uint32_t* __restrict__ n_contrib,
-                        float* __restrict__ out)
+                        float* __restrict__ out, uint2* __restrict__ bmask)
 {
     // Forward needs no cross-pixel communication, so every lane walks the list of ITS OWN pixel:
     // a lane only ever touches Gaussians whose alpha >= 1/255 footprint (conservatively) contains
@@ -302,7 +321,7 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
             gh_cp_async_commit();
             if (base + 2 * GH_CHUNK + tid < n) next_id = (uint32_t)inst[(size_t)rg.x + base + 2 * GH_CHUNK + tid];
         }
-        gh_build_pixel_lists(st, pixbits, buf, cnt, warp, lane, tx0, ty0);
+        gh_build_pixel_lists(st, pixbits, buf, cnt, warp, lane, tx0, ty0, bmask + rg.x + base);
         __syncthreads();
 
         if (!done) {
@@ -356,19 +375,22 @@ gh_blend_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __rest
 }
 
 // ------------------------------------------------------------------------------------------ backward
-// Backward staging: ONE window of GH_BWD_CHUNK instances (single-buffered; the other resident CTAs of
-// the SM cover the gather latency).  The 16 blocks of a warp walk their lists in lock-step, so a warp
-// spends max(list length over its blocks) steps per window: a wide window wastes fewer lanes on that
-// maximum than several narrow ones (tools/imbalance.py), and 384 records still leave room for 5 CTAs per SM.
+// Backward staging: ONE window of GH_BWD_CHUNK list positions at a time (single-buffered; the other resident
+// CTAs of the SM cover the gather latency).  Only the LIVE records of the window are staged -- those whose
+// block mask from the forward (gh_build_pixel_lists) is not zero -- packed into the first slots in list
+// order.  The 16 blocks of a warp walk their lists in lock-step, so a warp spends max(list length over its
+// blocks) steps per window: a wide window wastes fewer lanes on that maximum than several narrow ones
+// (tools/imbalance.py), and 384 records still leave room for 5 CTAs per SM.
 struct GhStageB {
-    float4 g0[GH_BWD_CHUNK];
+    float4 g0[GH_BWD_CHUNK];                 // [slot]
     float4 g1[GH_BWD_CHUNK];
     float2 feat[GH_BWD_CHUNK * GH_HALF_C];
-    uint32_t id[GH_BWD_CHUNK];
+    uint2 ref[GH_BWD_CHUNK];                 // [slot] (Gaussian id, list position)
+    uint2 mask[GH_BWD_CHUNK];                // [position - window base] block mask written by the forward
     uint32_t bits[GH_BWD_BLOCKS][GH_BWD_CHUNK / 32 + 1];   // [block][word]; +1 pad against bank conflicts
 };
 
-__device__ __forceinline__ void gh_stage_issue_b(GhStageB& st, int slot, uint32_t id,
+__device__ __forceinline__ void gh_stage_issue_b(GhStageB& st, int slot, uint32_t id, uint32_t pos,
                                                  const GhGeo* __restrict__ geo, const float* __restrict__ features) {
     const float4* gp = reinterpret_cast<const float4*>(geo + id);
     gh_cp_async16(&st.g0[slot], gp);
@@ -376,73 +398,43 @@ __device__ __forceinline__ void gh_stage_issue_b(GhStageB& st, int slot, uint32_
     const float2* fp = reinterpret_cast<const float2*>(features + (size_t)id * GH_NUM_CHANNELS);
 #pragma unroll
     for (int k = 0; k < GH_HALF_C; k++) gh_cp_async8(&st.feat[slot * GH_HALF_C + k], fp + k);
-    st.id[slot] = id;
+    st.ref[slot] = make_uint2(id, pos);
 }
 
-// Which of the tile's 64 blocks (2x2 pixels; bit = by * 8 + bx, .x = block rows 0..3, .y = rows 4..7)
-// can this Gaussian reach with alpha >= 1/255?  Exact-conservative: on each pixel row the set
-// {q(d) <= 2(thr+slack)} is an x-interval obtained from the quadratic; the interval is widened by
-// 0.01 px and rounded outwards to whole pixels.  Returns all ones when the conic is not positive
-// definite (no bound available).  Skipping a Gaussian in a block whose bit is clear cannot change any
-// pixel of that block: each of them would take the reference's `alpha < 1/255 -> continue`
-// (forward.cu:370, backward.cu:503).  Two pixel rows (one block row) per instruction; a row without a
-// real span has disc <= 0 -> s = NaN -> fminf / fmaxf ignore it.
-__device__ __forceinline__ uint2 gh_block_mask_2x2(const float4 g0, const float4 g1, float tx0, float ty0) {
-    const float gx = g0.x, gy = g0.y, a = g0.z, b = g0.w, c = g1.x, thr = g1.z, pd = g1.w;
-    if (pd == 0.f) return make_uint2(0xffffffffu, 0xffffffffu);
-    const float mxd = fmaxf(fabsf(gx - tx0), fabsf(gx - (tx0 + 15.f)));
-    const float myd = fmaxf(fabsf(gy - ty0), fabsf(gy - (ty0 + 15.f)));
-    const float slack = 1e-3f + 2e-5f * (a * mxd * mxd + c * myd * myd + 2.f * fabsf(b) * mxd * myd);
-    const float Q = 2.f * (thr + slack);
-    if (!(Q >= 0.f)) return (Q != Q) ? make_uint2(0xffffffffu, 0xffffffffu) : make_uint2(0u, 0u);
-    const float2 ia = gh_f2(__frcp_rn(a)), aQ = gh_f2(a * Q), bbac = gh_f2(b * b - a * c), gx2 = gh_f2(gx), b2 = gh_f2(b);
-    float2 dy = make_float2(gy - ty0, gy - (ty0 + 1.f));     // rows 2 by, 2 by + 1
-    uint32_t m[2] = {0u, 0u};
+// Live records of a window: ball[i] = which of the positions base + 32 i + [0, 32) are live.  Returns how many
+// live records lie before window position p (0 <= p <= GH_BWD_CHUNK) = the slot of position p when it is live.
+#define GH_BWD_BATCHES (GH_BWD_CHUNK / 32)
+__device__ __forceinline__ uint32_t gh_live_before(const uint32_t (&ball)[GH_BWD_BATCHES], int p) {
+    const int bi = p >> 5;
+    const uint32_t part = (1u << (p & 31)) - 1u;
+    uint32_t c = 0;
 #pragma unroll
-    for (int by = 0; by < 8; by++) {
-        // a dx^2 + 2 b dy dx + (c dy^2 - Q) <= 0,  dx = gx - px
-        const float2 disc = gh_fma2(gh_mul2(dy, dy), bbac, aQ);
-        const float2 s = gh_mul2(disc, make_float2(rsqrtf(disc.x), rsqrtf(disc.y)));   // NaN unless disc > 0
-        const float2 hb = gh_mul2(b2, dy);
-        const float2 lo2 = gh_fma2(gh_sub2(hb, s), ia, gx2), hi2 = gh_fma2(gh_add2(hb, s), ia, gx2);
-        const float xlo = fminf(fminf(1e30f, lo2.x), lo2.y), xhi = fmaxf(fmaxf(-1e30f, hi2.x), hi2.y);
-        // tile-local integer pixel columns inside [xlo - .01, xhi + .01]
-        const float lo = (xlo - 0.01f) - tx0, hi = (xhi + 0.01f) - tx0;
-        const int p0 = max(0, __float2int_ru(lo)), p1 = min(15, __float2int_rd(hi));
-        if (p0 <= p1) {
-            const int b0 = p0 >> 1, b1 = p1 >> 1;
-            m[by >> 2] |= (((2u << (b1 - b0)) - 1u) << b0) << (8 * (by & 3));
-        }
-        dy = gh_add2(dy, gh_f2(-2.f));
-    }
-    return make_uint2(m[0], m[1]);
+    for (int i = 0; i < GH_BWD_BATCHES; i++)
+        c += __popc(i < bi ? ball[i] : (i == bi ? (ball[i] & part) : 0u));
+    return c;
 }
 
-// batch `word` = instances [32 word, 32 word + 32) of the window, one per lane; two 5-step shuffle
-// transposes turn the 32 block masks into one list word per block (lane = block `lane` and block
-// 32 + lane).  The word is cut at the block's deepest blended list position `glast` here, once, rather
-// than in the traversal loop.
-__device__ __forceinline__ uint32_t gh_valid_bits(uint32_t glast, int first_pos) {
-    const int lim = (int)glast - first_pos;
+// batch `word` = slots [32 word, 32 word + 32) of the window, one per lane; two 5-step shuffle transposes turn
+// the 32 block masks into one list word per block (lane = block `lane` and block 32 + lane).  The word is cut at
+// the block's deepest blended list position here, once, rather than in the traversal loop: cut_lo / cut_hi =
+// the number of staged slots whose position lies before that of block `lane` / of block 32 + lane (positions
+// increase with the slot, so the cut is a prefix of the window).
+__device__ __forceinline__ uint32_t gh_valid_bits(uint32_t cut, int first_slot) {
+    const int lim = (int)cut - first_slot;
     return lim >= 32 ? 0xffffffffu : (lim <= 0 ? 0u : ((1u << lim) - 1u));
 }
 
-// glast_lo / glast_hi: deepest blended list position of block `lane` / of block 32 + lane
-__device__ __forceinline__ void gh_build_lists_b(GhStageB& st, int cnt, int word, int lane, float tx0, float ty0,
-                                                 int base, uint32_t glast_lo, uint32_t glast_hi) {
+__device__ __forceinline__ void gh_build_lists_b(GhStageB& st, int nlive, int word, int lane, int base,
+                                                 uint32_t cut_lo, uint32_t cut_hi) {
     const int j = word * 32 + lane;
     uint2 m = make_uint2(0u, 0u);
-    if (j < cnt) m = gh_block_mask_2x2(st.g0[j], st.g1[j], tx0, ty0);
+    if (j < nlive) m = st.mask[st.ref[j].y - (uint32_t)base];
     uint32_t lo = 0, hi = 0;
     if (__any_sync(0xffffffffu, m.x != 0u)) lo = gh_transpose32(m.x, lane);
     if (__any_sync(0xffffffffu, m.y != 0u)) hi = gh_transpose32(m.y, lane);
-    st.bits[lane][word] = lo & gh_valid_bits(glast_lo, base + word * 32);
-    st.bits[32 + lane][word] = hi & gh_valid_bits(glast_hi, base + word * 32);
+    st.bits[lane][word] = lo & gh_valid_bits(cut_lo, word * 32);
+    st.bits[32 + lane][word] = hi & gh_valid_bits(cut_hi, word * 32);
 }
-
-// Per-lane record of the reduction buffer, in float4.  gh_group2_reduce16 uses 3 of the 5 (the buffer
-// still has the size of an earlier 4-lane reduction; shrinking it changes the launch's shared memory).
-#define GH_RED_STRIDE4 5
 
 // The even lane keeps components 0..7, the odd lane 8..15 (two REDG.E.ADD.F32x4 each).  Each lane
 // stores the half its partner keeps (2 STS.128), loads the partner's contribution to its own half (2 LDS.128) and
@@ -554,20 +546,20 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
                          const GhGeo* __restrict__ geo, const float* __restrict__ features,
                          int W, int H, int gx, const float* __restrict__ bg,
                          const float* __restrict__ final_T, const uint32_t* __restrict__ n_contrib,
-                         const float* __restrict__ dL_dpix,
+                         const float* __restrict__ dL_dpix, const uint2* __restrict__ bmask,
                          float* __restrict__ acc16)   // [P][16]: colors 0..9, mean2D x,y, conic x,y,w, opacity
 {
     extern __shared__ __align__(16) unsigned char gh_bwd_smem[];
     GhStageB& st = *reinterpret_cast<GhStageB*>(gh_bwd_smem);
-    float4* red_buf = reinterpret_cast<float4*>(gh_bwd_smem + sizeof(GhStageB)) + (threadIdx.x >> 5) * 32 * GH_RED_STRIDE4;
+    float4* red_buf = reinterpret_cast<float4*>(gh_bwd_smem + sizeof(GhStageB)) + (threadIdx.x >> 5) * 32 * GH_RED2_STRIDE4;
     __shared__ uint32_t s_warp_last[GH_BWD_THREADS / 32];
     __shared__ uint32_t s_glast[GH_BWD_BLOCKS];              // per block: deepest list position any of its pixels blended
     __shared__ uint8_t s_perm[GH_BWD_THREADS / 32][GH_BWD_BLOCKS];   // per warp (redundant copies): rank -> block
+    __shared__ uint32_t s_ball[GH_BWD_BATCHES];              // live records of the window being staged (gh_live_before)
 
     const int tile = (int)tile_perm[blockIdx.x];      // heaviest tiles first
     const int tx = tile % gx, ty = tile / gx;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const float tx0 = (float)(tx * GH_BLOCK_X), ty0 = (float)(ty * GH_BLOCK_Y);
     const size_t plane = (size_t)H * W;
     const uint2 rg = ranges[tile];
 
@@ -595,32 +587,71 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
     const int nchunks = (n + GH_BWD_CHUNK - 1) / GH_BWD_CHUNK;
     if (nchunks == 0) return;
     constexpr int PER_THREAD = GH_BWD_CHUNK / GH_BWD_THREADS;
+    constexpr int WARPS = GH_BWD_THREADS / 32;
     // the builder's lane == block after the transposes: blocks `lane` and `32 + lane`
     const uint32_t glast_lo = s_glast[lane];
     const uint32_t glast_hi = s_glast[32 + lane];
+    const uint32_t* ids = reinterpret_cast<const uint32_t*>(inst + rg.x);   // low word of a record = Gaussian id
+    const uint2* masks = bmask + rg.x;
 
-    // ---- stage the last window (windows are visited last to first) and build its lists
+    // Thread tid covers window positions base + tid + 128 h (batch h * 4 + warp of s_ball).  The ids of the next
+    // window wait in registers; its masks (st.mask) and live ballots (s_ball) are published as soon as the
+    // current window's lists are built.
     uint32_t next_id[PER_THREAD];
-    {
-        const int base = (nchunks - 1) * GH_BWD_CHUNK;
-        const int cnt = n - base;
+    uint2 next_m[PER_THREAD];
+    auto fetch = [&](int base, int cnt) {
 #pragma unroll
         for (int h = 0; h < PER_THREAD; h++) {
-            const int slot = tid + h * GH_BWD_THREADS;
-            if (slot < cnt) gh_stage_issue_b(st, slot, (uint32_t)inst[(size_t)rg.x + base + slot], geo, features);
+            const int p = tid + h * GH_BWD_THREADS;
+            next_id[h] = 0u;
+            next_m[h] = make_uint2(0u, 0u);
+            if (p < cnt) { next_id[h] = ids[2 * (size_t)(base + p)]; next_m[h] = masks[base + p]; }
+        }
+    };
+    auto publish = [&]() {
+#pragma unroll
+        for (int h = 0; h < PER_THREAD; h++) {
+            st.mask[tid + h * GH_BWD_THREADS] = next_m[h];
+            const uint32_t b = __ballot_sync(0xffffffffu, (next_m[h].x | next_m[h].y) != 0u);
+            if (lane == 0) s_ball[h * WARPS + warp] = b;
+        }
+    };
+    // After a __syncthreads that follows publish(): stage the live records of window [base, base + GH_BWD_CHUNK)
+    // and build its per-block lists.  Returns the number of live records = staged slots.
+    auto stage = [&](int base, bool prefetch) -> int {
+        uint32_t ball[GH_BWD_BATCHES];
+#pragma unroll
+        for (int i = 0; i < GH_BWD_BATCHES; i++) ball[i] = s_ball[i];
+#pragma unroll
+        for (int h = 0; h < PER_THREAD; h++) {
+            const int p = tid + h * GH_BWD_THREADS;
+            if ((s_ball[h * WARPS + warp] >> lane) & 1u)
+                gh_stage_issue_b(st, (int)gh_live_before(ball, p), next_id[h], (uint32_t)(base + p), geo, features);
         }
         gh_cp_async_commit();
-        if (nchunks > 1) {
-#pragma unroll
-            for (int h = 0; h < PER_THREAD; h++)
-                next_id[h] = (uint32_t)inst[(size_t)rg.x + base - GH_BWD_CHUNK + tid + h * GH_BWD_THREADS];
-        }
+        const int nlive = (int)gh_live_before(ball, GH_BWD_CHUNK);
+        const uint32_t b0 = (uint32_t)base;
+        const uint32_t cut_lo = gh_live_before(ball, (int)min(max(glast_lo, b0) - b0, (uint32_t)GH_BWD_CHUNK));
+        const uint32_t cut_hi = gh_live_before(ball, (int)min(max(glast_hi, b0) - b0, (uint32_t)GH_BWD_CHUNK));
+        if (prefetch) fetch(base - GH_BWD_CHUNK, GH_BWD_CHUNK);
         gh_cp_async_wait_all();
         __syncthreads();
-        for (int word = warp; word * 32 < cnt; word += GH_BWD_THREADS / 32)
-            gh_build_lists_b(st, cnt, word, lane, tx0, ty0, base, glast_lo, glast_hi);
+        // per-block lists: each of the 4 warps transposes every fourth batch of 32 staged records
+        for (int word = warp; word * 32 < nlive; word += WARPS)
+            gh_build_lists_b(st, nlive, word, lane, base, cut_lo, cut_hi);
+        __syncthreads();
+        if (prefetch) publish();        // st.mask and s_ball are free again
+        return nlive;
+    };
+
+    // ---- stage the last window (windows are visited last to first) and build its lists
+    {
+        const int base = (nchunks - 1) * GH_BWD_CHUNK;
+        fetch(base, n - base);
+        publish();
         __syncthreads();
     }
+    int nlive = stage((nchunks - 1) * GH_BWD_CHUNK, nchunks > 1);
 
     // ---- block -> (warp, lane group) assignment.  The blocks of a warp advance in lock-step, so a warp pays for
     // its LONGEST list: blocks are ranked by the length of their list in the window just built (lane b counts block
@@ -628,7 +659,7 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
     // neighbours of that ranking.  Any assignment gives the same gradients up to the order of the float atomics.
     int blk;
     {
-        const int nw = (n - (nchunks - 1) * GH_BWD_CHUNK + 31) >> 5;
+        const int nw = (nlive + 31) >> 5;
         uint32_t len0 = 0, len1 = 0;
         for (int w = 0; w < nw; w++) {
             len0 += __popc(st.bits[lane][w]);
@@ -691,27 +722,13 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
 
     for (int c = nchunks - 1; c >= 0; c--) {
         const int base = c * GH_BWD_CHUNK;
-        const int cnt = min(GH_BWD_CHUNK, n - base);
         if (c != nchunks - 1) {
             __syncthreads();                       // everyone is done with the previous window
-#pragma unroll
-            for (int h = 0; h < PER_THREAD; h++) gh_stage_issue_b(st, tid + h * GH_BWD_THREADS, next_id[h], geo, features);
-            gh_cp_async_commit();
-            if (c > 0) {
-#pragma unroll
-                for (int h = 0; h < PER_THREAD; h++)
-                    next_id[h] = (uint32_t)inst[(size_t)rg.x + base - GH_BWD_CHUNK + tid + h * GH_BWD_THREADS];
-            }
-            gh_cp_async_wait_all();
-            __syncthreads();
-            // per-block lists: each of the 4 warps scan-converts every fourth batch of 32 Gaussians
-            for (int word = warp; word * 32 < cnt; word += GH_BWD_THREADS / 32)
-                gh_build_lists_b(st, cnt, word, lane, tx0, ty0, base, glast_lo, glast_hi);
-            __syncthreads();
+            nlive = stage(base, c > 0);
         }
         if ((uint32_t)base >= wlast) continue;
 
-        int wi = (cnt + 31) >> 5;
+        int wi = (nlive + 31) >> 5;
         uint32_t cur = 0;
         while (true) {
             while (cur == 0 && wi > 0) cur = st.bits[blk][--wi];
@@ -722,10 +739,11 @@ gh_blend_backward_kernel(const uint2* __restrict__ ranges, const uint32_t* __res
             const int bpos = act ? 31 - __clz(cur) : 0;   // back to front
             cur &= ~(1u << bpos);
             const int jj = act ? wi * 32 + bpos : 0;
-            const uint32_t id = st.id[jj];
+            const uint2 rf = st.ref[jj];
+            const uint32_t id = rf.x;
             const float4 g0 = st.g0[jj], g1 = st.g1[jj];
             const float2* feat = &st.feat[jj * GH_HALF_C];
-            const uint32_t pos = act ? (uint32_t)(base + jj) : 0xffffffffu;
+            const uint32_t pos = act ? rf.y : 0xffffffffu;
             float v[16];
             const bool contrib = gh_bwd_pair(pr, g0, g1, feat, pxf, pos, ddelx_dx, ddely_dy, v);
             const uint32_t cm = __ballot_sync(0xffffffffu, contrib);
@@ -778,24 +796,27 @@ void gh_launch_blend_forward(int W, int H, int gx, int gy, GhGeomWS geom, GhImgW
                              const float* features, const float* bg, float* out_color,
                              cudaStream_t stream)
 {
-    // ask for the largest shared-memory carve-out so that 4 CTAs (4 x 48 KB) are resident per SM
+    // ask for the largest shared-memory carve-out so that 4 CTAs (4 x 48 KB) are resident per SM.
+    // The block masks for the backward go to bin.tmp: the long-list sort (gh_tile_split_long_kernel /
+    // gh_segment_sort_kernel) uses it as scratch, but that ran to completion before this launch on the same stream.
     const int smem = (int)(sizeof(GhStage) + (GH_CHUNK / 32) * 256 * sizeof(uint32_t));
     cudaFuncSetAttribute(gh_blend_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     cudaFuncSetAttribute(gh_blend_forward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     gh_blend_forward_kernel<<<gx * gy, 256, smem, stream>>>(img.ranges, img.tile_perm, bin.inst, geom.geo, features,
-                                                         W, H, gx, bg, img.final_T, img.n_contrib, out_color);
+                                                         W, H, gx, bg, img.final_T, img.n_contrib, out_color,
+                                                         reinterpret_cast<uint2*>(bin.tmp));
 }
 
 void gh_launch_blend_backward(int W, int H, int gx, int gy, GhGeomWS geom, GhImgWS img, GhBinWS bin,
                               const float* features, const float* bg, const float* dL_dpix,
                               cudaStream_t stream)
 {
-    const int smem = (int)(sizeof(GhStageB) + GH_BWD_THREADS * GH_RED_STRIDE4 * sizeof(float4));
+    const int smem = (int)(sizeof(GhStageB) + GH_BWD_THREADS * GH_RED2_STRIDE4 * sizeof(float4));
     cudaFuncSetAttribute(gh_blend_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     cudaFuncSetAttribute(gh_blend_backward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     gh_blend_backward_kernel<<<gx * gy, GH_BWD_THREADS, smem, stream>>>(img.ranges, img.tile_perm, bin.inst, geom.geo, features,
                                                           W, H, gx, bg, img.final_T, img.n_contrib, dL_dpix,
-                                                          geom.acc16);
+                                                          reinterpret_cast<const uint2*>(bin.tmp), geom.acc16);
 }
 
 void gh_launch_unpack_grads(int P, GhGeomWS geom, float* dL_dmean2D, float* dL_dconic, float* dL_dopacity,

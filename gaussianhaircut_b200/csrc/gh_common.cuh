@@ -100,7 +100,8 @@ struct GhImgWS {
 
 struct GhBinWS {
     uint64_t* inst;   // [R]  (depth_bits << 32 | gaussian_idx), bucketed by tile, sorted within a tile
-    uint64_t* tmp;    // [R]  scratch of the long-list sort (MSD split target)
+    uint64_t* tmp;    // [R]  scratch of the long-list sort (MSD split target); then, written by the forward blend,
+                      //      the backward block mask of each record at its list position (gh_blend.cu)
     uint2* seg;       // [R/768 + R/2048 + 2] (start, length) of the split segments
     static __host__ __device__ size_t max_segments(size_t R) { return R / 768 + R / 2048 + 2; }
     static __host__ __device__ size_t bytes(size_t R) {
